@@ -1,7 +1,7 @@
 """Benchmark of the volumetric-render hot path (BASELINE.json: rays/s @ 64 samples/ray).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c3|c4|c5]
-                  [--precision tc_fp16x3|tc_fp16|fp32] [--dense]
+                  [--precision tc_fp16x3|tc_fp16|fp32] [--dense] [--dump-outputs DIR]
 
 Default (`--config c2`, the configuration BASELINE.json's metric is quoted on): a "step" = one pass of the hot path over
 one synthetic batch: at N=1 ONE 512x512 all-hit view of the synth-313 body (BASELINE.json configs[1]: single B200,
@@ -14,6 +14,10 @@ per-GPU work is fixed (262 144 rays per step) => "scaling": "weak".
 `e2e`    : the same metric through the public API make_renderer(cfg, net).render(batch) with the batch in PINNED HOST
            memory: H2D of rays/near/far/pose per step, prepare_sp_input, weight pack, render, D2H of rgb_map + depth_map
            (at N>1: of the GATHERED frame, on the view's owner rank v % N, each GPU using its own PCIe link) inside the timed region.
+`--dump-outputs DIR` (c2): after the timed steps, the frame the last timed step rendered (its last view) as
+           DIR/{rgb_map,disp_map,acc_map,depth_map}.npy, float32, (1, 262144[, 3]) in ray order; disp_map holds 0 instead of
+           the renderer's NaN on rays with acc_map == 0.  The inputs are built from fixed seeds, so two builds run with the
+           same arguments can be compared output for output.
 `--impl reference`: the reference's own CPU implementation of the path (the oracle port of /root/reference's
            if_clight_renderer + latent_xyzc + raw2outputs, validated bit-exact against the unmodified reference in the
            build container), all host threads, each step a bounded sample (--ref-rays rays) of the same workload.
@@ -328,6 +332,16 @@ def time_steps(args, dev, world, step_fn, before_step=None):
     return sum(step_ms), step_ms
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one float32 .npy per output the timed path returned."""
+    import numpy as np
+    host = {k: v.detach().float().contiguous().cpu().numpy() for k, v in arrays.items()}
+    assert sum(a.nbytes for a in host.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def max_over_ranks(vals, dev, world):
     import torch.distributed as dist
     t = torch.tensor(vals, dtype=torch.float64, device=dev)
@@ -400,6 +414,13 @@ def run_c2(args, rank, world, local_rank):
     launches = ren.launches - launches0[0]
     stats = [int(v) for v in ren.stats.tolist()]
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        gatherer.drain()
+        out = nbdist.slab_views(gatherer.frames[(gatherer.v - 1) % gatherer.depth])
+        # raw2outputs gives disp_map = 1 / max(1e-10, 0 / 0) = NaN on rays that cross no density (acc_map == 0); such a
+        # ray sees nothing, i.e. is infinitely far: disparity 0.  Any other non-finite value is written as it is.
+        out["disp_map"] = torch.where(out["acc_map"] == 0, torch.zeros_like(out["disp_map"]), out["disp_map"])
+        dump_outputs(args.dump_outputs, out)
 
     # ---- e2e through the public API with host buffers: per view H2D of this rank's rays (+ the frame's pose tensors) from
     # pinned memory, Renderer.render, the gather, and the D2H of the GATHERED frame on the view's owner (rank v % N)
@@ -976,9 +997,15 @@ def main():
     ap.add_argument("--c5-size", type=int, default=1024, help="c5: image side")
     ap.add_argument("--train-precision", default="tc_tf32x3", choices=["tc_tf32x3", "fp32"], help="c3: precision of the gradient path")
     ap.add_argument("--importance", type=int, default=128, help="c3: importance samples of the fine pass (0 = coarse only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="c2: write the outputs of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = {"c2": 20, "c3": 20, "c4": 2, "c5": 3}[args.config]
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl, args.config) != ("b200", "c2"):
+        ap.error("--dump-outputs is implemented for the default configuration (--config c2) of the b200 implementation")
     args.warmup = max(3, args.warmup) if args.impl == "b200" else max(1, args.warmup)
     if args.config in ("c4", "c5") and args.impl == "b200":
         args.warmup = min(args.warmup, 3)

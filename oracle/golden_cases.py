@@ -29,11 +29,12 @@ CASES = {
 }
 
 
-def build_case(name):
-    """-> (scene, render_kwargs incl. t_rand) with rays subsampled by the case's stride."""
+def build_case(name, rescale=None):
+    """-> (scene, render_kwargs incl. t_rand) with rays subsampled by the case's stride.
+    rescale: the (s0, spread) pair the case's golden vectors were generated with (synth.make_scene)."""
     from oracle import synth
     skw, rkw, stride = CASES[name]
-    scene = synth.make_scene(**skw)
+    scene = synth.make_scene(**skw, rescale=rescale)
     n = scene["ray_o"].shape[1]
     idx = torch.arange(0, n, stride)
     for k in ("ray_o", "ray_d", "near", "far"):
@@ -59,10 +60,10 @@ HIER_CASES = {
 }
 
 
-def build_hier_case(name):
+def build_hier_case(name, rescale=None):
     from oracle import synth
     skw, rkw, stride = HIER_CASES[name]
-    scene = synth.make_scene(**skw)
+    scene = synth.make_scene(**skw, rescale=rescale)
     idx = torch.arange(0, scene["ray_o"].shape[1], stride)
     for k in ("ray_o", "ray_d", "near", "far"):
         scene[k] = scene[k][:, idx].contiguous()

@@ -9,9 +9,9 @@ GRAD_KEYS = ["fc_0.weight", "fc_0.bias", "fc_1.weight", "fc_1.bias", "fc_2.weigh
 N_SAMPLES = 32
 
 
-def build():
+def build(rescale=None):
     from oracle import synth
-    scene = synth.make_scene(H=24, W=24, scale=0.25, all_hit=True, latent_index=3)
+    scene = synth.make_scene(H=24, W=24, scale=0.25, all_hit=True, latent_index=3, rescale=rescale)
     idx = torch.arange(0, scene["ray_o"].shape[1], 5)
     for k in ("ray_o", "ray_d", "near", "far"):
         scene[k] = scene[k][:, idx].contiguous()
@@ -43,10 +43,10 @@ def oracle_grads(scene, t_rand, G):
 N_IMPORTANCE = 48
 
 
-def hier_build():
+def hier_build(rescale=None):
     """Same scene / jitter as build(), plus the uniforms of sample_pdf and a cotangent for the coarse image (the trainer adds
     img_loss0 on rgb0, lib/train/trainers/if_nerf_clight.py:29-32)."""
-    scene, t_rand, G = build()
+    scene, t_rand, G = build(rescale)
     B, n = scene["ray_o"].shape[:2]
     g = torch.Generator().manual_seed(100)
     u = torch.rand((B, n, N_IMPORTANCE), generator=g)

@@ -4,7 +4,8 @@ on the seeded synthetic cases of oracle/golden_cases.py.  Run in the build conta
     python -m oracle.make_golden
 
 Each file holds the reference's five outputs (fp32) plus a sha256 of every input tensor, so a
-consumer on another machine can prove it rebuilt the identical inputs from the seeds.
+consumer on another machine can prove it rebuilt the identical inputs from the seeds and from the case's
+calibration pair in tests/golden/rescale.json.
 TEST INFRASTRUCTURE ONLY."""
 import os
 import sys
@@ -40,6 +41,7 @@ def main():
         print("%-22s rays=%-5d acc.mean=%.3f nan_disp=%d -> %s (%d KB)" % (
             name, acc.numel(), float(acc.mean()), int(torch.isnan(ret["disp_map"]).sum()), path,
             os.path.getsize(path) // 1024))
+        record_rescale(name, scene)
 
 
 def data_golden():
@@ -114,6 +116,7 @@ def grad_golden():
         arrays["abs:vol%d" % l] = np.float64(v.grad.double().abs().sum())
     path = os.path.join(ROOT, "tests", "golden", "grad_train_s32.npz")
     np.savez_compressed(path, **arrays)
+    record_rescale("grad_train_s32", scene)
     print("gradient fingerprints ->", path, "|dfc_0.weight|_1 = %.4e" % float(arrays["abs:fc_0.weight"]))
 
 
@@ -133,6 +136,7 @@ def hier_golden():
         print("%-22s rays=%-5d acc.mean=%.3f |rgb - rgb0|max=%.3f -> %s (%d KB)" % (
             name, ret["acc_map"].numel(), float(ret["acc_map"].mean()), float((ret["rgb_map"] - ret["rgb0"]).abs().max()),
             path, os.path.getsize(path) // 1024))
+        record_rescale(name, scene)
 
 
 def hier_grad_golden():
@@ -156,11 +160,39 @@ def hier_grad_golden():
         arrays["abs:vol%d" % l] = np.float64(v.grad.double().abs().sum())
     path = os.path.join(ROOT, "tests", "golden", "grad_hier_s32_i48.npz")
     np.savez_compressed(path, **arrays)
+    record_rescale("grad_hier_s32_i48", scene)
     print("hierarchical gradient fingerprints ->", path, "|dfc_0.weight|_1 = %.4e" % float(arrays["abs:fc_0.weight"]))
 
 
+def module_keys_golden():
+    """state_dict keys of the reference's SparseConvNet (latent_xyzc.py:166-274, spconv stubbed, so only its
+    BatchNorm1d entries), which the dense encoder has to reproduce for checkpoints to load."""
+    import json
+    from oracle import ref_harness
+    _, latent_xyzc, _, _ = ref_harness.load_reference()
+    keys = sorted(latent_xyzc.SparseConvNet().state_dict())
+    path = os.path.join(ROOT, "tests", "golden", "sparseconvnet_keys.json")
+    with open(path, "w") as f:
+        json.dump(keys, f, indent=0)
+        f.write("\n")
+    print("SparseConvNet state_dict keys ->", path, "(%d)" % len(keys))
+
+
+def record_rescale(name, scene):
+    """Record the (s0, spread) pair case `name` was generated with (synth.make_scene, key "rescale") in
+    tests/golden/rescale.json: measured on another host, its last bit can differ and the inputs with it."""
+    import json
+    path = os.path.join(ROOT, "tests", "golden", "rescale.json")
+    table = json.load(open(path)) if os.path.exists(path) else {}
+    table[name] = list(scene["rescale"])
+    with open(path, "w") as f:
+        f.write("{\n" + ",\n".join('  "%s": [%r, %r]' % (k, v[0], v[1]) for k, v in sorted(table.items())) + "\n}\n")
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "data":
+    if len(sys.argv) > 1 and sys.argv[1] == "keys":
+        module_keys_golden()
+    elif len(sys.argv) > 1 and sys.argv[1] == "data":
         data_golden()
     elif len(sys.argv) > 1 and sys.argv[1] == "only":      # python -m oracle.make_golden only <case> ...: render cases by name
         main()
@@ -169,6 +201,7 @@ if __name__ == "__main__":
         hier_grad_golden()
     else:
         data_golden()
+        module_keys_golden()
         grad_golden()
         main()
         hier_golden()

@@ -311,10 +311,10 @@ def _mlp_sigma(w, feats):
     return h @ w["alpha_fc.weight"][:, :, 0].t() + w["alpha_fc.bias"]
 
 
-def trained_like_rescale(w, volumes, seed=313, sigma_empty=-10.0, sigma_p95=30.0, rgb_gain=20.0):
-    """Rescale alpha_fc / rgb_fc so the random net behaves like a trained one
-    (SURVEY 7 hard parts 2-3): all-zero features give sigma = sigma_empty exactly
-    (robustly negative => no far-plane sign flips), active features reach ~+30."""
+def rescale_stats(w, volumes, seed=313):
+    """(s0, spread) that trained_like_rescale calibrates on: sigma of all-zero features and the 95th percentile of
+    sigma(active) - s0, as float32 values.  They come out of float32 matmuls, so their last bit depends on the
+    host's BLAS; golden cases pass the values their vectors were generated with to make_scene (`rescale`)."""
     g = torch.Generator().manual_seed(seed + 3)
     # feature samples: random active voxels of each level, concatenated channel-wise
     feats = []
@@ -330,6 +330,15 @@ def trained_like_rescale(w, volumes, seed=313, sigma_empty=-10.0, sigma_p95=30.0
     s_act = _mlp_sigma(w, feats)[:, 0]
     s0 = _mlp_sigma(w, torch.zeros(1, 352))[0, 0]
     spread = torch.quantile(s_act - s0, 0.95).clamp_min(1e-6)
+    return float(s0), float(spread)
+
+
+def trained_like_rescale(w, stats, sigma_empty=-10.0, sigma_p95=30.0, rgb_gain=20.0):
+    """Rescale alpha_fc / rgb_fc so the random net behaves like a trained one
+    (SURVEY 7 hard parts 2-3): all-zero features give sigma = sigma_empty exactly
+    (robustly negative => no far-plane sign flips), active features reach ~+30.
+    stats: the (s0, spread) pair of rescale_stats."""
+    s0, spread = (torch.tensor(v, dtype=torch.float32) for v in stats)
     s = float((sigma_p95 - sigma_empty) / spread)
     w = dict(w)
     w["alpha_fc.weight"] = w["alpha_fc.weight"] * s
@@ -341,7 +350,8 @@ def trained_like_rescale(w, volumes, seed=313, sigma_empty=-10.0, sigma_p95=30.0
 # ----------------------------------------------------------------------------- scene
 def make_scene(seed=313, H=512, W=512, scale=1.0, voxel_size=(0.005, 0.005, 0.005), all_hit=True,
                num_train_frame=60, latent_index=0, n_rays=None, azimuth_deg=20.0,
-               Rh=(0.3, -0.2, 0.1), Th=(0.1, 0.2, 1.0), th_shape=(1, 3), batch=1, ray_box_pad=0.15, volume_seed=None):
+               Rh=(0.3, -0.2, 0.1), Th=(0.1, 0.2, 1.0), th_shape=(1, 3), batch=1, ray_box_pad=0.15, volume_seed=None,
+               rescale=None):
     """Build the batch dict of multi_view_dataset.py:157-180 (as default_collate would
     hand it to Renderer.render) + dense volumes + decoder weights.
 
@@ -354,15 +364,19 @@ def make_scene(seed=313, H=512, W=512, scale=1.0, voxel_size=(0.005, 0.005, 0.00
     (multi_view_dataset.py:78-80); 15 cm keeps the last sample of every ray in
     exactly-empty space, so sigma_last = sigma(empty) < 0 robustly and the 1e10 last
     interval of raw2outputs (nerf_net_utils.py:23-26) cannot flip alpha between
-    implementations."""
+    implementations.
+    rescale: (s0, spread) for trained_like_rescale instead of measuring them on this host; the scene
+    records the pair it used under "rescale"."""
     verts = humanoid_vertices(seed, N_SMPL_VERTS, scale)
     Rm = _rodrigues(Rh)
     world = (verts.astype(np.float64) @ Rm.T + np.asarray(Th, np.float64) * 1.0).astype(np.float32)
     coord, out_sh, can_bounds, bounds, R, Th_f = prepare_input(world, Rh, Th, voxel_size)
     # volume_seed: other feature values on the same body (the frames of a multi-pose batch share the decoder, not the volume)
     volumes, fracs = make_volumes(coord, out_sh, seed if volume_seed is None else volume_seed)
-    weights = trained_like_rescale(make_weights(seed, num_train_frame), make_volumes(coord, out_sh, seed)[0]
-                                   if volume_seed is not None else volumes, seed)
+    w0 = make_weights(seed, num_train_frame)
+    if rescale is None:
+        rescale = rescale_stats(w0, make_volumes(coord, out_sh, seed)[0] if volume_seed is not None else volumes, seed)
+    weights = trained_like_rescale(w0, rescale)
 
     ray_box = can_bounds.copy()
     ray_box[0] -= ray_box_pad
@@ -394,6 +408,7 @@ def make_scene(seed=313, H=512, W=512, scale=1.0, voxel_size=(0.005, 0.005, 0.00
         "mask_at_box": torch.from_numpy(np.stack(masks, 0)),
         "volumes": volumes, "weights": weights, "voxel_size": [float(v) for v in voxel_size],
         "active_fraction": fracs, "H": H, "W": W, "verts_world": torch.from_numpy(world),
+        "rescale": tuple(rescale),
     }
     return scene
 

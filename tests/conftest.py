@@ -1,3 +1,4 @@
+import json
 import os
 import sys
 
@@ -35,6 +36,13 @@ def load_golden(name):
     return out
 
 
+def golden_rescale(name):
+    """The (s0, spread) pair the golden vectors `name` were generated with (oracle/synth.py rescale_stats): measured
+    again here, its last bit would follow this host's BLAS and the inputs would no longer be the golden ones."""
+    with open(os.path.join(GOLDEN_DIR, "rescale.json")) as f:
+        return tuple(json.load(f)[name])
+
+
 _case_cache = {}
 
 
@@ -44,7 +52,7 @@ def golden_case(name):
     if name not in _case_cache:
         from oracle import synth
         from oracle import golden_cases
-        scene, rkw = golden_cases.build_case(name)
+        scene, rkw = golden_cases.build_case(name, golden_rescale(name))
         gold = load_golden(name)
         assert synth.scene_checksum(scene) == gold["input_sha256"], (
             "rebuilt inputs differ from the ones the golden vectors were generated on "
@@ -59,7 +67,7 @@ def hier_golden_case(name):
     if key not in _case_cache:
         from oracle import synth
         from oracle import golden_cases
-        scene, rkw = golden_cases.build_hier_case(name)
+        scene, rkw = golden_cases.build_hier_case(name, golden_rescale(name))
         gold = load_golden(name)
         assert synth.scene_checksum(scene) == gold["input_sha256"], "rebuilt inputs differ from the golden generator's"
         _case_cache[key] = (scene, rkw, gold)

@@ -5,14 +5,20 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import load_golden
+from conftest import golden_rescale, load_golden
 from oracle import grad_case
+
+# The fingerprints come from the reference's float32 autograd on one host.  Float32 GEMMs round differently in the last
+# bits on another CPU, BLAS code path or thread count; the reference's own autograd there misses the fingerprints by as
+# much as the oracle does (the two agree bit for bit on any one host).  A sum that cancels heavily, or an entry far
+# below the tensor's typical size, magnifies that rounding, so each relative bound is taken against the magnitude that
+# was summed: the tensor's L1 norm for its sum, its mean |entry| for a single entry.
 
 
 @pytest.fixture(scope="module")
 def case():
     from oracle import synth
-    scene, t_rand, G = grad_case.build()
+    scene, t_rand, G = grad_case.build(golden_rescale("grad_train_s32"))
     gold = load_golden("grad_train_s32")
     assert synth.scene_checksum(scene) == gold["input_sha256"]
     pg, vg, ret = grad_case.oracle_grads(scene, t_rand, G)
@@ -24,9 +30,11 @@ def test_oracle_autograd_matches_reference_fingerprints(case):
     for k in grad_case.GRAD_KEYS:
         g = pg[k]
         assert g is not None, k
-        np.testing.assert_allclose(float(g.double().sum()), float(gold["sum:" + k]), rtol=1e-5, atol=1e-6, err_msg=k)
+        np.testing.assert_allclose(float(g.double().sum()), float(gold["sum:" + k]), rtol=1e-5,
+                                   atol=1e-6 + 1e-5 * float(gold["abs:" + k]), err_msg=k)
         np.testing.assert_allclose(float(g.double().abs().sum()), float(gold["abs:" + k]), rtol=1e-5, err_msg=k)
-        np.testing.assert_allclose(g.reshape(-1)[:64].numpy(), gold["head:" + k], rtol=1e-4, atol=1e-6, err_msg=k)
+        np.testing.assert_allclose(g.reshape(-1)[:64].numpy(), gold["head:" + k], rtol=1e-4,
+                                   atol=1e-6 + 1e-4 * float(gold["abs:" + k]) / g.numel(), err_msg=k)
     for l, g in enumerate(vg):
         np.testing.assert_allclose(float(g.double().abs().sum()), float(gold["abs:vol%d" % l]), rtol=1e-5)
     assert float(pg["fc_0.weight"].abs().sum()) > 1.0          # not vacuous
@@ -95,7 +103,7 @@ def test_inference_path_unchanged_under_no_grad(case):
 @pytest.fixture(scope="module")
 def hier_case():
     from oracle import synth
-    scene, t_rand, u, G = grad_case.hier_build()
+    scene, t_rand, u, G = grad_case.hier_build(golden_rescale("grad_hier_s32_i48"))
     gold = load_golden("grad_hier_s32_i48")
     assert synth.scene_checksum(scene) == gold["input_sha256"]
     pg, vg, ret = grad_case.oracle_hier_grads(scene, t_rand, u, G)
@@ -107,9 +115,11 @@ def test_hierarchical_oracle_autograd_matches_reference_fingerprints(hier_case):
     scene, t_rand, u, G, pg, vg, ret, gold = hier_case
     for k in grad_case.GRAD_KEYS:
         g = pg[k]
-        np.testing.assert_allclose(float(g.double().sum()), float(gold["sum:" + k]), rtol=1e-5, atol=1e-6, err_msg=k)
+        np.testing.assert_allclose(float(g.double().sum()), float(gold["sum:" + k]), rtol=1e-5,
+                                   atol=1e-6 + 1e-5 * float(gold["abs:" + k]), err_msg=k)
         np.testing.assert_allclose(float(g.double().abs().sum()), float(gold["abs:" + k]), rtol=1e-5, err_msg=k)
-        np.testing.assert_allclose(g.reshape(-1)[:64].numpy(), gold["head:" + k], rtol=1e-4, atol=1e-6, err_msg=k)
+        np.testing.assert_allclose(g.reshape(-1)[:64].numpy(), gold["head:" + k], rtol=1e-4,
+                                   atol=1e-6 + 1e-4 * float(gold["abs:" + k]) / g.numel(), err_msg=k)
     for l, g in enumerate(vg):
         np.testing.assert_allclose(float(g.double().abs().sum()), float(gold["abs:vol%d" % l]), rtol=1e-5)
 

@@ -12,16 +12,26 @@ from oracle import golden_cases, neuralbody_oracle as O
 KEYS = ("rgb_map", "disp_map", "acc_map", "weights", "depth_map")
 
 
+# The oracle performs the reference's torch ops in the same order, so on any one host the two agree bit for bit.  The
+# golden vectors were made on one host; float32 GEMMs round differently in the last bits on another CPU, BLAS code path
+# or thread count, and volume rendering magnifies that.  Bound on |oracle - golden| relative to the output's largest
+# magnitude (the reference itself, run on another host, reaches 1e-4 on hier_s64_i128's z_vals).
+F32_HOST_TOL = 5e-4
+
+
+def _assert_matches_golden(a, b, k):
+    assert a.shape == b.shape, k
+    np.testing.assert_array_equal(np.isnan(a), np.isnan(b), err_msg=k)      # NaNs (acc == 0 rays) at the same rays
+    a, b = np.nan_to_num(a), np.nan_to_num(b)
+    np.testing.assert_allclose(a, b, rtol=0, atol=F32_HOST_TOL * float(np.abs(b).max()), err_msg=k)
+
+
 @pytest.mark.parametrize("name", list(golden_cases.CASES))
 def test_oracle_matches_reference_golden(name):
     scene, rkw, gold = golden_case(name)
     out = O.render_mmsk(scene, **rkw) if "masks" in rkw else O.render(scene, **rkw)
     for k in KEYS:
-        a, b = out[k].numpy(), gold[k]
-        assert a.shape == b.shape
-        # same torch ops in the same order => bit-identical, NaNs (acc == 0 rays) included
-        np.testing.assert_array_equal(np.isnan(a), np.isnan(b))
-        np.testing.assert_array_equal(np.nan_to_num(a), np.nan_to_num(b), err_msg=k)
+        _assert_matches_golden(out[k].numpy(), gold[k], k)
 
 
 @pytest.mark.parametrize("name", list(golden_cases.HIER_CASES))
@@ -30,10 +40,7 @@ def test_hierarchical_oracle_matches_reference_pieces(name):
     scene, rkw, gold = hier_golden_case(name)
     out = O.render_hierarchical(scene, **rkw)
     for k in KEYS + ("rgb0", "disp0", "acc0", "z_std", "z_vals"):
-        a, b = out[k].numpy(), gold[k]
-        assert a.shape == b.shape, k
-        np.testing.assert_array_equal(np.isnan(a), np.isnan(b))
-        np.testing.assert_array_equal(np.nan_to_num(a), np.nan_to_num(b), err_msg=k)
+        _assert_matches_golden(out[k].numpy(), gold[k], k)
     S, Ni = rkw["n_samples"], rkw["n_importance"]
     assert gold["z_vals"].shape[-1] == S + Ni and (np.diff(gold["z_vals"], axis=-1) >= 0).all()
     assert np.abs(gold["rgb_map"] - gold["rgb0"]).max() > 1e-3      # the fine pass is not a no-op on these scenes

@@ -1,9 +1,12 @@
 """CPU: f-2(ii) -- the dense-PyTorch emulation of the reference's SparseConvNet encode against a brute-force sparse
 restatement of spconv's semantics (oracle/spconv_oracle.py).  PARITY UNPINNED against spconv itself: it is not in the image."""
+import json
+import os
+
 import numpy as np
-import pytest
 import torch
 
+from conftest import GOLDEN_DIR
 from neuralbody_b200.lib.networks.sparse_encode import DenseSparseConvNet, _Block
 from oracle import spconv_oracle as SO
 
@@ -89,13 +92,10 @@ def test_network_hook_and_gradients():
 
 
 def test_reference_module_tree_has_the_same_batchnorm_keys():
-    """In the build container: the reference's SparseConvNet (spconv stubbed) exposes its BatchNorm1d entries under the same
-    names, i.e. the Sequential child indices agree (conv 0/3/6, bn 1/4/7)."""
-    from oracle import ref_harness
-    if not ref_harness.reference_available():
-        pytest.skip("needs /root/reference")
-    _, latent_xyzc, _, _ = ref_harness.load_reference()
-    ref_keys = {k for k in latent_xyzc.SparseConvNet().state_dict()}
+    """The reference's SparseConvNet (spconv stubbed; keys stored by `python -m oracle.make_golden keys`) exposes its
+    BatchNorm1d entries under the same names, i.e. the Sequential child indices agree (conv 0/3/6, bn 1/4/7)."""
+    with open(os.path.join(GOLDEN_DIR, "sparseconvnet_keys.json")) as f:
+        ref_keys = set(json.load(f))
     ours = {k for k in DenseSparseConvNet().state_dict() if ".weight" not in k or k.split(".")[1] in ("1", "4", "7")}
     ours = {k for k in ours if k.split(".")[1] in ("1", "4", "7")}
     assert ref_keys == ours and len(ours) == 17 * 5          # 17 conv + BatchNorm1d + ReLU triples
