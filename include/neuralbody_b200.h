@@ -226,6 +226,35 @@ int nb_gen_rays_sharded(const nb_camera* cam, int rank, int world, int chunk, in
                         float* ray_o /* device (n_local,3) */, float* ray_d, float* near, float* far,
                         unsigned char* mask_at_box /* device (n_local) */, void* stream);
 
+/* f-3, surface extraction of the mesh renderer (lib/networks/renderer/if_mesh_renderer.py:46-47):
+ *     cube = np.pad(cube, pad, mode='constant'); vertices, triangles = mcubes.marching_cubes(cube, isovalue)
+ * on a device grid, with the padding virtual (corners outside the data read 0; vertex coordinates are in padded index space).
+ * Convention: corners v0..v7 = (x,y,z) (x+1,y,z) (x+1,y+1,z) (x,y+1,z) and the same four at z+1; bit m of a cell's case is
+ * set iff cube[v_m] <= isovalue (fp32 compare); Bourke's edge / triangle tables; one vertex per crossed lattice edge, shared
+ * by every cell touching it, at p_lower + t e_axis, t = (iso - f_lower) / (f_upper - f_lower) in fp32.
+ * Output order (deterministic, no atomics): vertices by (flat padded index of the edge's lower endpoint, axis x < y < z);
+ * triangles by (flat padded index of the cell's lower corner, triangle-table order), vertex ids in table order.
+ * Usage: nb_mcubes_count writes the two totals to device counts[2] and leaves the scanned offsets in the workspace;
+ * nb_mcubes_emit must follow it on the same stream with the same arguments and workspace. */
+typedef struct nb_mcubes_args {
+    const float* cube;     /* device (nx, ny, nz) fp32, C order (z fastest): numpy's cube[i, j, k] */
+    int nx, ny, nz;
+    float isovalue;        /* cfg.mesh_th */
+    int pad;               /* >= 0: virtual zero padding on every side (upstream: 10) */
+    void* workspace;       /* device scratch of nb_mcubes_workspace_bytes(nx, ny, nz, pad) bytes */
+    size_t workspace_bytes;
+} nb_mcubes_args;
+
+/* Host arithmetic only (no CUDA call); 0 for non-positive dimensions or pad < 0. */
+size_t nb_mcubes_workspace_bytes(int nx, int ny, int nz, int pad);
+/* counts: device int[2] = (n_vertices, n_triangles).  NB_ERR_UNSUPPORTED for grids whose worst case (5 triangles per
+ * cell, 3 vertices per lattice point) overflows int32 indices. */
+int nb_mcubes_count(const nb_mcubes_args* args, int* counts, void* stream);
+/* vertices: device (max_vertices, 3) fp32; triangles: device (max_triangles, 3) int32; writes beyond either capacity are
+ * dropped (size them from nb_mcubes_count's counts). */
+int nb_mcubes_emit(const nb_mcubes_args* args, float* vertices, int* triangles, int max_vertices, int max_triangles,
+                   void* stream);
+
 /* number of kernels nb_render_fwd enqueues per FRAME of a call: 1 for NB_PRECISION_FP32 (the single fused exact kernel),
  * 3 for the tensor-core inference precisions (classify, decoder, composite; plus one 32-byte memset per call), 9 for
  * NB_PRECISION_TC_TF32X3 (colour-matrix build, classify, gather, 4 GEMMs, rgb head, composite). */

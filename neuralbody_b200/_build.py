@@ -9,7 +9,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libneuralbody_b200.so")
-SOURCES = ["nb_capi.cu", "nb_render_f32.cu", "nb_render_tc_list.cu", "nb_tc_probe.cu", "nb_tc_probe2.cu", "nb_tc_bench.cu", "nb_render_bwd.cu", "nb_train.cu", "nb_sample_pdf.cu"]
+SOURCES = ["nb_capi.cu", "nb_render_f32.cu", "nb_render_tc_list.cu", "nb_tc_probe.cu", "nb_tc_probe2.cu", "nb_tc_bench.cu", "nb_render_bwd.cu", "nb_train.cu", "nb_sample_pdf.cu", "nb_mcubes.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 OBJ_DIR = os.path.join(HERE, "build")
 

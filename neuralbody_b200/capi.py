@@ -14,7 +14,8 @@ NB_NUM_LEVELS = 4
 EXPORTS = ["nb_abi_version", "nb_last_error", "nb_has_precision", "nb_packed_volume_bytes", "nb_packed_volume_level_offset",
            "nb_pack_volume", "nb_packed_weights_bytes", "nb_pack_weights", "nb_render_fwd",
            "nb_render_fwd_launches", "nb_render_fwd_workspace_bytes", "nb_debug_tc_probe", "nb_debug_tc_probe2", "nb_debug_mma_rate", "nb_render_bwd", "nb_render_save_bytes",
-           "nb_render_bwd_workspace_bytes", "nb_render_save_bytes_for", "nb_render_bwd_workspace_bytes_for", "nb_debug_gemm_tf32x3", "nb_decode_density", "nb_gen_rays", "nb_gen_rays_sharded", "nb_sample_pdf"]
+           "nb_render_bwd_workspace_bytes", "nb_render_save_bytes_for", "nb_render_bwd_workspace_bytes_for", "nb_debug_gemm_tf32x3", "nb_decode_density", "nb_gen_rays", "nb_gen_rays_sharded", "nb_sample_pdf",
+           "nb_mcubes_workspace_bytes", "nb_mcubes_count", "nb_mcubes_emit"]
 
 
 class nb_volume_level(C.Structure):
@@ -68,6 +69,11 @@ class nb_render_bwd_args(C.Structure):
         ("weights", C.POINTER(nb_decoder_weights)), ("grads", C.POINTER(nb_decoder_weights)),
         ("d_volumes", C.c_void_p * NB_NUM_LEVELS), ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t),
     ]
+
+
+class nb_mcubes_args(C.Structure):
+    _fields_ = [("cube", C.c_void_p), ("nx", C.c_int), ("ny", C.c_int), ("nz", C.c_int), ("isovalue", C.c_float),
+                ("pad", C.c_int), ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
 
 
 _lib = None
@@ -124,6 +130,12 @@ def load(path=None):
     lib.nb_gen_rays_sharded.argtypes = [C.POINTER(nb_camera)] + [C.c_int] * 4 + [C.c_void_p] * 6
     lib.nb_sample_pdf.restype = C.c_int
     lib.nb_sample_pdf.argtypes = [C.POINTER(nb_importance_args), C.c_void_p]
+    lib.nb_mcubes_workspace_bytes.restype = C.c_size_t
+    lib.nb_mcubes_workspace_bytes.argtypes = [C.c_int] * 4
+    lib.nb_mcubes_count.restype = C.c_int
+    lib.nb_mcubes_count.argtypes = [C.POINTER(nb_mcubes_args), C.c_void_p, C.c_void_p]
+    lib.nb_mcubes_emit.restype = C.c_int
+    lib.nb_mcubes_emit.argtypes = [C.POINTER(nb_mcubes_args), C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
     lib.nb_debug_tc_probe.restype = C.c_int
     lib.nb_debug_tc_probe.argtypes = [C.c_void_p] * 5 + [C.c_int, C.c_void_p]
     lib.nb_debug_tc_probe2.restype = C.c_int

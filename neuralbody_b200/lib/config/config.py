@@ -7,6 +7,7 @@ the yaml-only keys of configs/snapshot_exp/snapshot_f3c.yaml:55-78):
   xyz_res, view_res                               embedder.py:53-54
   num_train_frame                                 latent_xyzc.py:16
   H, W, ratio, N_rand, chunk
+  mesh_th                                         if_mesh_renderer.py:47
   network_module/path, renderer_module/path       make_network.py / make_renderer.py
 Same yaml format (`parent_cfg` inheritance, config.py:149-152) and the same trailing
 `KEY VALUE` override form (config.py:153).  Unlike upstream nothing is parsed from
@@ -102,6 +103,8 @@ def _defaults():
     c.num_train_frame = 60
     c.voxel_size = [0.005, 0.005, 0.005]
     c.big_box = False
+    # mesh extraction (config.py:44-45; the 313 / snapshot yamls set 5 in mesh_cfg)
+    c.mesh_th = 50
     # B200 renderer options (new)
     c.render_precision = "tc_fp16x3"    # "fp32" exact FFMA kernel | "tc_fp16x3" tcgen05, 3-pass hi/lo density path
                                         # (meets the 1e-3 parity gate) | "tc_fp16" tcgen05 1-pass (fastest, ~4e-3 on depth)
